@@ -5,6 +5,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...      # the reference-shaped CPU fan-out on the host cores
+    python bench.py ... --dump-outputs DIR    # also write the last timed step's forecasts to DIR/*.npy
 
 A "step" is one pass of the hot path over one batch of synthetic series:
   value : device-resident y[N,T] -> forecast table, kernels + (N>1) one NCCL all_gather, timed with
@@ -14,6 +15,7 @@ A "step" is one pass of the hot path over one batch of synthetic series:
 One JSON line on stdout (rank 0).  See DESIGN.md section 5 for how each field is measured.
 """
 import argparse
+import atexit
 import json
 import os
 import statistics
@@ -73,7 +75,16 @@ def parse():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--ref-groups", type=int, default=0, help="groups per step of the reference arm (0 = 16 x cores)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the forecast table of the last timed step to DIR/forecast.npy "
+                         "(and the e2e leg's last host output to DIR/e2e_forecast.npy), float32; tables larger than "
+                         "30 MB are reduced to a fixed seeded sample of rows, the same on every run with the same arguments")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
+    return args
 
 
 def peaks():
@@ -82,6 +93,26 @@ def peaks():
         with open(p) as f:
             return float(json.load(f)["hbm_gbs"]), "measured (MEASURED_PEAKS.json hbm_gbs)"
     return 6650.0, "fallback (B200_PROFILING.md 6.65 TB/s)"
+
+
+DUMP_BYTES = 30_000_000      # per dumped table: forecast.npy and e2e_forecast.npy stay under 64 MB together
+
+
+def dump_output(dirname, name, table):
+    """Write ``table`` (rows x columns, torch tensor or NumPy array) to dirname/name.npy as float32, so that two builds
+    of the project can be compared output for output.  A table over DUMP_BYTES keeps a fixed sample of its rows
+    (numpy default_rng(0), in row order): the same rows on every run of the same shape."""
+    import numpy as np
+    import torch
+    rows, cols = table.shape
+    keep = max(1, DUMP_BYTES // (4 * cols))
+    if rows > keep:
+        idx = np.sort(np.random.default_rng(0).choice(rows, keep, replace=False))
+        table = table[torch.from_numpy(idx).to(table.device)] if torch.is_tensor(table) else table[idx]
+    if torch.is_tensor(table):
+        table = table.cpu().numpy()
+    os.makedirs(dirname, exist_ok=True)
+    np.save(os.path.join(dirname, f"{name}.npy"), np.ascontiguousarray(table, dtype=np.float32))
 
 
 class ClockSampler:
@@ -97,6 +128,7 @@ class ClockSampler:
         try:
             self.proc = subprocess.Popen(["nvidia-smi", f"--query-gpu={self.Q}", "--format=csv,noheader,nounits",
                                           "-i", str(self.index), "-lms", "20"], stdout=subprocess.PIPE, text=True)
+            atexit.register(self.proc.kill)     # the sampler never outlives the bench, even when a step raises
             self.th = threading.Thread(target=self._read, daemon=True)
             self.th.start()
         except OSError:
@@ -476,6 +508,8 @@ def run_ours(args):
         dist.all_reduce(tt, op=dist.ReduceOp.MAX)
     total_ms, kern_ms_avg = float(tt[0]), float(tt[1])
     clocks = sampler.stop(wall0, wall1) if rank == 0 else None
+    if args.dump_outputs and rank == 0:                 # the table as the last timed step left it (every rank's is equal)
+        dump_output(args.dump_outputs, "forecast", table)
     value = world * n * K / (total_ms * 1e-3)
     gather_check = None
     shard_only = None
@@ -556,6 +590,8 @@ def run_ours(args):
         if world > 1:
             dist.all_reduce(tte, op=dist.ReduceOp.MAX)
         te = float(tte[0])
+        if args.dump_outputs and rank == 0:
+            dump_output(args.dump_outputs, "e2e_forecast", oh)
         chk = float(np.abs(oh[:4096] - table[rank * n: rank * n + 4096].cpu().numpy()).max())
         e2e = {"value": world * ne * Ke / te, "unit": UNIT, "h2d_bytes_per_step": int(h2d_actual),
                "d2h_bytes_per_step": ne * h * 4, "series_per_step_per_gpu": ne, "steps": Ke,
